@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- boosting rounds/sec on synthetic 10M x 100 (BASELINE.json metric, config C3).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is one boosting round (gradient -> all tree levels -> prediction-cache update, including
@@ -11,6 +11,8 @@ quantised matrix resident in HBM; `e2e` goes through the xgb.train() replacement
 (upload + GPU sketch/binning + K rounds + a per-round metric read-back, all inside the timed region).
 `--impl reference` times the CPU path (the oracle port of XGBoost hist; `xgboost` itself is not
 installable here) on the host cores for the same config.
+`--dump-outputs DIR` writes, after the timed steps, what the timed path computed in its last step (see dump_outputs);
+the synthetic inputs depend on the arguments only, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -259,6 +261,32 @@ def parity_check(E, args, rank, world, dm_kw, bst_timed, dm_timed):
     return out
 
 
+TREE_FIELDS = ("left", "right", "parent", "split_feature", "split_bin", "split_cond", "default_left", "value",
+               "base_weight", "loss_chg", "sum_hess", "split_type", "cat_bits")
+DUMP_MARGIN_VALUES = 12_000_000     # float32: 48 MB, which keeps a dump (trees included) under 64 MB
+
+
+def dump_outputs(out_dir, trees, margin):
+    """Write the outputs of one boosting round as .npy files (float32 / float64) under out_dir:
+    tree_<field>.npy -- the node arrays of the trees the round added, concatenated in tree order (integer fields as
+                        float64, which holds them exactly); tree_nodes.npy -- the node count of each of those trees;
+    margin.npy       -- the training margin (prediction cache) after the round, rows x outputs; above
+                        DUMP_MARGIN_VALUES values only the rows of a fixed sample (numpy default_rng(0), sorted)."""
+    files = {"tree_nodes": np.array([len(t["left"]) for t in trees], np.float64)}
+    for k in TREE_FIELDS:
+        a = np.concatenate([np.asarray(t[k]) for t in trees])
+        files["tree_" + k] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    m = np.asarray(margin, np.float32)
+    m = m.reshape(m.shape[0], -1)
+    if m.size > DUMP_MARGIN_VALUES:
+        rows = np.random.default_rng(0).choice(m.shape[0], DUMP_MARGIN_VALUES // m.shape[1], replace=False)
+        m = m[np.sort(rows)]
+    files["margin"] = m
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in files.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def measured_peak():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -302,6 +330,9 @@ def run_reference(args, rank, world):
     for _ in range(args.steps):
         bst.boost(bins, y)
     dt = time.time() - t0
+    if args.dump_outputs:
+        trees = [bst.tree(i) for i in range(bst.num_trees - bst.K, bst.num_trees)]
+        dump_outputs(args.dump_outputs, [{k: getattr(t, k) for k in TREE_FIELDS} for t in trees], bst.margin)
     v = args.steps / dt
     line = {"impl": "reference", "metric": "boosting rounds/sec", "value": v, "unit": "rounds/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True,
@@ -333,7 +364,12 @@ def main():
                     help="synthetic data generator: numpy on the host, or torch Philox on the GPU (default for > 2e9 values)")
     ap.add_argument("--no-public-e2e", action="store_true", help="skip the end-to-end run through train(RayDMatrix, RayParams)")
     ap.add_argument("--profile", type=int, default=1, help="2 = per-phase CUDA-event timers (adds event records)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the trees of the last step and the training margin as .npy files "
+                         "(rank 0; with several ranks, the margin of rank 0's rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     wl = WORKLOADS[args.workload]
@@ -415,6 +451,10 @@ def main():
         hist_ms = max_over_ranks(timers["hist_ms"])
         ms_per_step = 1e3 * wall / args.steps
         value = args.steps / wall
+        if args.dump_outputs and rank == 0:
+            n_trees, per_round = bst.num_trees(), bst.num_class * bst.num_parallel_tree
+            dump_outputs(args.dump_outputs, [bst.get_tree(i) for i in range(n_trees - per_round, n_trees)],
+                         bst.predict(dm, output_margin=True, training=True))
         final_metric = bst.eval_set([(dm, "train")], 0).split("\t", 1)[-1]
         exchange_kind = "none (1 GPU)" if world == 1 else ("nccl" if os.environ.get("B2_EXCHANGE", "").lower() == "nccl" else "nvlink peer memory (nccl if peers cannot be mapped)")
         parity = None if args.no_parity else parity_check(E, args, rank, world, dm_kw, bst, dm)

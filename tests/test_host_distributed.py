@@ -16,6 +16,9 @@ def use_cpu_engine(monkeypatch):
     import xgboost_ray_b200.main as M
     import xgboost_ray_b200.xgb as seam
     monkeypatch.setenv("OMP_NUM_THREADS", "1")
+    # the stand-in computes on the CPU: the host layer and its actors see no GPU, as on a CPU-only machine, also where
+    # CUDA_VISIBLE_DEVICES names one (the host layer would otherwise assign it to the actors, one GPU each)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     monkeypatch.setattr(seam, "xgboost", ce)
     orig = M._validate_ray_params
 
